@@ -291,7 +291,28 @@ def run_reference(W, steps, warmup, sample_blocks=0):
 
 
 # ----------------------------------------------------------------------------- device-resident run
-def device_run(W, args, rank, world, local_rank, sharded, dist, steps, warmup, want_parity=True, flush_mb=256):
+DUMP_CAP = 1 << 19          # entries per dumped array (4 MiB in float64): a dump stays well below 64 MiB
+
+
+def dump_outputs(hp, S, dump_dir):
+    """Write what a caller of the iteration receives (oracle/gates.py device_outputs, plus the Lorentz vectors) as
+    dump_dir/<name>.npy in float64.  An array longer than DUMP_CAP is written as the entries at a fixed, seeded,
+    sorted sample of its indices, so two builds given the same arguments can be compared file by file."""
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    import gates
+    outs = gates.device_outputs(hp, S, int(S.L["L"].nnz))
+    if hp.nq:
+        outs.update(qblkmul=hp.q_y.cpu().numpy()[:hp.qdim], ddot=hp.q_dd.cpu().numpy()[:hp.nq],
+                    quadadd_hi=hp.r_hi.cpu().numpy()[:hp.m], quadadd_lo=hp.r_lo.cpu().numpy()[:hp.m])
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, a in outs.items():
+        a = np.asarray(a, dtype=np.float64).ravel()
+        if a.size > DUMP_CAP:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_CAP, replace=False))]
+        np.save(os.path.join(dump_dir, name + ".npy"), a)
+
+
+def device_run(W, args, rank, world, local_rank, sharded, dist, steps, warmup, want_parity=True, flush_mb=256, dump_dir=None):
     import torch
     from sedumi_b200 import device as sbdev
     S, d = W.S, W.d
@@ -374,6 +395,8 @@ def device_run(W, args, rank, world, local_rank, sharded, dist, steps, warmup, w
             ev[k][1].record(stream)
         barrier()
         out.wall = time.perf_counter() - t_wall0
+        if dump_dir and rank == 0:
+            dump_outputs(hp, S, dump_dir)
         launches = lib.sb200_kernel_launches() - l0
         if not args.no_graph:
             launches = hp.launches_per_iteration * steps      # kernels inside the replayed graphs
@@ -620,6 +643,8 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch kernels one by one instead of replaying a CUDA graph")
     ap.add_argument("--replicas", action="store_true", help="N>1: N independent replicas (weak scaling) instead of sharding")
     ap.add_argument("--ref-blocks", type=int, default=4, help="reference arm: PSD blocks in the per-step sample (0 = all)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64, at most 64 MiB)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
@@ -671,7 +696,7 @@ def main():
             return bytes(t.cpu().tolist())
         sbdev.comm_init(rank, world, local_rank, bcast)
     out = device_run(W, args, rank, world, local_rank, sharded, dist if world > 1 else None, args.steps, args.warmup,
-                     want_parity=not args.no_parity)
+                     want_parity=not args.no_parity, dump_dir=args.dump_outputs)
     config["parallelism"] = out.parallelism if sharded else (f"replicas x{world} (no data-path collective)" if world > 1 else "1 GPU")
     value = (1 if sharded else world) * args.steps / (out.ms_max * 1e-3)
     line = {"metric": METRIC, "value": value, "unit": "iterations/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,

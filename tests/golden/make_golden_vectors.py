@@ -77,4 +77,21 @@ save("ada_small_mixed", At=csc(S.At), Ablkjc=S.Ablkjc, lqperm=S.Aord["lqperm"], 
      dz=csc(S.Aord["dz"]), ADApat=csc(S.ADA), K_l=K["l"], K_q=K["q"], K_s=K["s"],
      d_l=d["l"], d_det=d["det"], d_q1=d["q1"], d_q2=d["q2"], d_u=d["u"], d_perm=d["perm"],
      udsqr=udsqr, ADA=ADA.data, absd=absd)
+
+# ---- host-side structures: what the reference's own MEX files make of the same inputs (tests/test_host.py)
+dbg = refpath.ref_dir(debug=True)
+for name in ("arch0", "control07", "nb", "trto3"):
+    At, b, c, K = problems.internal_problem(name)
+    S = setup.build_setup(At, b, c, K)
+    sperm, dz = dbg.incorder(S.At, S.Ablkjc[:, 2], K["mainblks"][2], nlhs=2)
+    save(f"host_setup_{name}", Ablkjc=dbg.partitA(S.At, K["mainblks"].reshape(1, -1)), sperm=sperm, dz=csc(dz))
+Xf = random_sparse_spd(300, 0.01, 2)
+Lf = symbolic.symbolic_factor(Xf)
+save("host_symbolic_fill300", nnzL=ref.symfctmex(Xf, ref.ordmmdmex(Xf))["L"].nnz, tmpsiz=dbg.choltmpsiz(Lf).ravel()[0])
+for seed, nd in ((4, 3), (8, 4)):
+    raw = problems.synth_blockdiag_sdp(nblk=4, n=10, m=48, nlink=6, density=0.08, dense_lp=nd, seed=seed)
+    At, b, c, K = cones.pretransfo(*raw)[:4]
+    S = setup.build_setup(At, b, c, K, denf=0.3, perm=np.arange(At.shape[1]))
+    sym = refpath.DenseColumnRef(S, dict(S.L)).sym
+    save(f"host_symbcholden_seed{seed}", LAD=csc(sym["LAD"]), dz=csc(sym["dz"]), perm=sym["perm"], first=sym["first"])
 print("golden vectors written to", OUT, sorted(os.listdir(OUT)))

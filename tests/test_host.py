@@ -3,10 +3,8 @@ import numpy as np
 import pytest
 import scipy.sparse as sp
 
-from helpers import dbg, ref
+import golden_io
 from sedumi_b200.host import cones, problems, setup, symbolic
-
-needs_ref = pytest.mark.skipif(not ref.has("partitA"), reason="oracle/_ref not built")
 
 
 def test_pretransfo_layout_control07():
@@ -52,14 +50,15 @@ def test_free_and_rotated_cones_reach_internal_form():
     assert K["l"] == 1 + 3 and At.shape[0] == K["N"]
 
 
-@needs_ref
 @pytest.mark.parametrize("name", ["arch0", "control07", "nb", "trto3"])
 def test_setup_matches_reference_mex(name):
+    """Ablkjc, sperm and dz against the reference's partitA and incorder on the same problem (stored outputs)."""
     At, b, c, K = problems.internal_problem(name)
     S = setup.build_setup(At, b, c, K)
-    assert np.array_equal(dbg.partitA(S.At, K["mainblks"].reshape(1, -1)), S.Ablkjc)
-    sperm, dz = dbg.incorder(S.At, S.Ablkjc[:, 2], K["mainblks"][2], nlhs=2)
-    assert np.array_equal(sperm.ravel(), S.Aord["sperm"].ravel())
+    g = golden_io.load(f"host_setup_{name}")
+    assert np.array_equal(g["Ablkjc"], S.Ablkjc)
+    assert np.array_equal(g["sperm"].ravel(), S.Aord["sperm"].ravel())
+    dz = g["dz"]
     assert np.array_equal(dz.indptr, S.Aord["dz"].indptr) and np.array_equal(dz.indices, S.Aord["dz"].indices)
     assert S.ADA.nnz == S.m * S.m and len(S.L["xsuper"]) == 2      # every shipped fixture: dense ADA, 1 supernode
 
@@ -82,14 +81,14 @@ def test_symbolic_factor_is_valid_and_supernodal(m, density):
             assert np.array_equal(ind[ip[j] + 1:ip[j + 1]], ind[ip[j + 1]:ip[j + 2]])
 
 
-@needs_ref
 def test_symbolic_matches_reference_fill():
+    """Fill against the reference's ordmmdmex + symfctmex, tmpsiz against its choltmpsiz (stored outputs)."""
     from helpers import random_sparse_spd
     X = random_sparse_spd(300, 0.01, 2)
     L = symbolic.symbolic_factor(X)
-    L2 = ref.symfctmex(X, ref.ordmmdmex(X))
-    assert abs(L["L"].nnz - L2["L"].nnz) <= 0.15 * L2["L"].nnz          # both minimum-degree orderings
-    assert L["tmpsiz"] == float(dbg.choltmpsiz(L).ravel()[0])
+    g = golden_io.load("host_symbolic_fill300")
+    assert abs(L["L"].nnz - int(g["nnzL"])) <= 0.15 * int(g["nnzL"])      # both minimum-degree orderings
+    assert L["tmpsiz"] == float(g["tmpsiz"])
 
 
 def test_scaling_generators_are_interior():
@@ -105,23 +104,17 @@ def test_scaling_generators_are_interior():
 
 def test_symbcholden_restatement_matches_reference_symbolic_chain():
     """host.symbolic.symbcholden (symbfwblk + incorder + finsymbden restated for LP dense columns) against the reference's
-    own symbolic MEX files (symbcholden.m:45-62)."""
-    import os
-    import sys
-    from helpers import ROOT
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import refpath
-    from sedumi_b200.host import symbolic
+    own symbolic MEX files (symbcholden.m:45-62; stored outputs of oracle/refpath.py's DenseColumnRef)."""
     for seed, nd in ((4, 3), (8, 4)):
         raw = problems.synth_blockdiag_sdp(nblk=4, n=10, m=48, nlink=6, density=0.08, dense_lp=nd, seed=seed)
         At, b, c, K = cones.pretransfo(*raw)[:4]
         S = setup.build_setup(At, b, c, K, denf=0.3, perm=np.arange(At.shape[1]))
         assert len(S.dense.cols) == nd
-        DC = refpath.DenseColumnRef(S, dict(S.L))
+        ref_sym = golden_io.load(f"host_symbcholden_seed{seed}")
         mine = symbolic.symbcholden(S.L, S.dense)
         for k in ("LAD", "dz"):
-            a, r = sp.csc_matrix(mine[k]), sp.csc_matrix(DC.sym[k])
+            a, r = sp.csc_matrix(mine[k]), ref_sym[k]
             a.sort_indices()
             assert np.array_equal(a.indptr, r.indptr) and np.array_equal(a.indices, r.indices), k
-        assert np.array_equal(mine["perm"].ravel(), np.asarray(DC.sym["perm"]).ravel())
-        assert np.array_equal(mine["first"].ravel(), np.asarray(DC.sym["first"]).ravel())
+        assert np.array_equal(mine["perm"].ravel(), np.asarray(ref_sym["perm"]).ravel())
+        assert np.array_equal(mine["first"].ravel(), np.asarray(ref_sym["first"]).ravel())
