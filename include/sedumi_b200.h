@@ -275,6 +275,38 @@ int sb200_wrappcg_dev(sb200_ada_plan *ada, sb200_psd_plan *psd, sb200_chol_plan 
                       const double *u_dev, const int *perm_dev, const double *Lrect_dev, const double *Ld_dev,
                       const int *flag_dev, const double *rv_dev, const double *rb_dev, double *y_dev, double *dx_dev,
                       double *r_dev, double *scal_dev, double *work_dev);
+/* The whole of wrapPcg.m:43-130 with loopPcg.m:53-170 (PopK.m:39-55, asmDxq.m:41-69, Amul.m:40-56 with LP dense
+ * columns): the direct step above, then PCG refinement while |r|_inf >= y0 * cgpars.restol.  Cones LP, Lorentz and
+ * real PSD; x layout [K.l | nq trace entries | norm-bound parts (qdim) | PSD], so N = K.l + sum(K.q) + sum(K.s.^2).
+ *   dpr1: the product-form factor of the LP dense columns (after sb200_dpr1fact_dev), NULL without dense columns;
+ *         Ld_dev is then the d that dpr1fact returned (deninfac.m), otherwise L.d.
+ *   cones->q1/q2 also refresh the plan's DAt.q (sb200_getdatm_dev), used by the residual update of every CG step.
+ *   Outputs y (m), dx (N), r (m) and *status: k = CG steps counted as wrapPcg counts them (0 when |D A' p| = 0, with
+ *   y = 0 and dx = rv), stop = STOP of the last loopPcg call (0: none ran), trials = refinement trials, normr = |r|_inf.
+ * The host side of the loop reads a few bytes back after the direct step and after every CG step (one synchronisation
+ * when the direct step already meets the tolerance), so the entry refuses to run while the library stream is being
+ * captured.  Dense Lorentz blocks are refused.  work_dev: sb200_wrappcg_full_work(N, m, nq, qdim) doubles. */
+typedef struct sb200_dpr1_plan sb200_dpr1_plan;     /* dense columns, see below */
+typedef struct {
+  double restol, stagtol;      /* cgpars.restol, cgpars.stagtol (checkpars.m:171-191: 5e-3, 5e-14) */
+  int maxiter, refine, qprec;  /* cgpars.maxiter, .refine, .qprec (49, 1, 1) */
+} sb200_cgpars;
+typedef struct {
+  sb_idx nq, qdim;             /* Lorentz cones, sum(K.q - 1) */
+  const long long *qbs_dev;    /* nq + 1 norm-bound block starts relative to the first norm-bound entry */
+  const double *det_dev, *q1_dev, *q2_dev, *auxdet_dev, *auxtr_dev;    /* d.det, d.q1, d.q2, d.auxdet, d.auxtr */
+  sb_idx nden;                 /* LP dense columns (dense.l) */
+  const int *den_cols_dev;     /* their 0-based positions in x (dense.cols - 1) */
+  const double *denA_dev;      /* dense.A, column-major m x nden */
+  sb_idx ndenq;                /* dense Lorentz blocks (dense.q): must be 0 */
+} sb200_pcg_cones;
+typedef struct { sb_idx k; int stop; int trials; double normr; } sb200_pcg_status;
+sb_idx sb200_wrappcg_full_work(sb_idx N, sb_idx m, sb_idx nq, sb_idx qdim);
+int sb200_wrappcg_full_dev(sb200_ada_plan *ada, sb200_psd_plan *psd, sb200_chol_plan *chol, sb200_dpr1_plan *dpr1,
+                           const sb200_pcg_cones *cones, const sb200_cgpars *cgpars, const double *dl_dev,
+                           const double *u_dev, const int *perm_dev, const double *Lrect_dev, const double *Ld_dev,
+                           const int *flag_dev, const double *rv_dev, const double *rb_dev, double y0, double *y_dev,
+                           double *dx_dev, double *r_dev, sb200_pcg_status *status, double *work_dev);
 int sb200_ada_plan_csr(sb200_ada_plan *plan, const long long **Ajc, const int **Air, const double **Apr,
                        const long long **rowptr, const int **rowcol, const int **rowsrc, sb_idx *N, sb_idx *m,
                        sb_idx *lpN, sb_idx *nq);
@@ -328,7 +360,6 @@ int sb200_dpr1solve(int backward, sb_idx m, sb_idx nrhs, sb_idx nden, const sb_i
 
 /* device-resident product form: plan from Lsymb (dz, perm, first; 0-based), factor from the dense block L\Ad (m x n,
  * column-major, rows in the factor's permuted order) and L.d, then in-place solves on m x nrhs device data */
-typedef struct sb200_dpr1_plan sb200_dpr1_plan;
 int  sb200_dpr1_plan_create(sb200_dpr1_plan **plan, sb_idx m, sb_idx n, const sb_idx *dzjc, const sb_idx *dzir,
                             const sb_idx *colperm, const sb_idx *firstpiv);
 void sb200_dpr1_plan_destroy(sb200_dpr1_plan *plan);

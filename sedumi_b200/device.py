@@ -47,6 +47,7 @@ def lib() -> C.CDLL:
         L.sb200_ada_plan_nnz.restype = I64
         L.sb200_psd_plan_lenud.restype = I64
         L.sb200_chol_plan_lb_dev.restype = VP
+        L.sb200_wrappcg_full_work.restype = I64
         _lib = L
     return _lib
 
@@ -88,7 +89,7 @@ EXPORTS = [
     "sb200_comm_unique_id", "sb200_comm_init_rank", "sb200_comm_size", "sb200_comm_rank", "sb200_comm_nccl_version",
     "sb200_comm_stats", "sb200_allreduce_sum_dev", "sb200_allreduce_sum2_dev", "sb200_comm_destroy",
     "sb200_blkchol_sharded_dev", "sb200_ldl_solve_sharded_dev",
-    "sb200_wrappcg_dev", "sb200_ldl_solve2_dev", "sb200_ada_plan_csr", "sb200_psd_plan_blocks",
+    "sb200_wrappcg_dev", "sb200_wrappcg_full_dev", "sb200_wrappcg_full_work", "sb200_ldl_solve2_dev", "sb200_ada_plan_csr", "sb200_psd_plan_blocks",
     "sb200_dpr1_plan_create", "sb200_dpr1_plan_destroy", "sb200_dpr1fact_dev", "sb200_dpr1solve_dev", "sb200_dpr1_plan_download",
     "sb200_gather_dev", "sb200_scale_by_d_dev", "sb200_chol_plan_lb_dev",
 ]
@@ -116,6 +117,21 @@ def comm_stats():
 
 class _CholPars(C.Structure):
     _fields_ = [("abstol", C.c_double), ("canceltol", C.c_double), ("maxu", C.c_double)]
+
+
+class CgPars(C.Structure):
+    """cgpars of wrapPcg / loopPcg; the defaults are checkpars.m:171-191."""
+    _fields_ = [("restol", C.c_double), ("stagtol", C.c_double), ("maxiter", C.c_int), ("refine", C.c_int), ("qprec", C.c_int)]
+    DEFAULTS = dict(restol=5e-3, stagtol=5e-14, maxiter=49, refine=1, qprec=1)
+
+
+class _PcgCones(C.Structure):
+    _fields_ = [("nq", I64), ("qdim", I64), ("qbs", VP), ("det", VP), ("q1", VP), ("q2", VP), ("auxdet", VP), ("auxtr", VP),
+                ("nden", I64), ("den_cols", VP), ("denA", VP), ("ndenq", I64)]
+
+
+class _PcgStatus(C.Structure):
+    _fields_ = [("k", I64), ("stop", C.c_int), ("trials", C.c_int), ("normr", C.c_double)]
 
 
 class HotPath:
@@ -168,6 +184,7 @@ class HotPath:
         q = np.asarray(K["q"], dtype=np.int64)
         self.qdim = int((q - 1).sum()) if self.nq else 0
         self.d_q1, self.d_q2 = z(self.nq), z(self.qdim)
+        self.d_auxdet, self.d_auxtr = z(self.nq), z(self.nq)
         if self.nq:
             bsq = np.r_[0, np.cumsum(q - 1)].astype(np.int64)
             self.qbs = torch.from_numpy(bsq).to(self.dev)
@@ -230,7 +247,8 @@ class HotPath:
         """Host -> device copy of the NT scaling; returns bytes moved."""
         t = self.torch
         nbytes = 0
-        for name, dst in (("l", self.d_l), ("det", self.d_det), ("u", self.d_u), ("q1", self.d_q1), ("q2", self.d_q2)):
+        for name, dst in (("l", self.d_l), ("det", self.d_det), ("u", self.d_u), ("q1", self.d_q1), ("q2", self.d_q2),
+                          ("auxdet", self.d_auxdet), ("auxtr", self.d_auxtr)):
             if name not in d:
                 continue
             a = np.ascontiguousarray(np.asarray(d[name], dtype=np.float64).ravel())
@@ -460,6 +478,49 @@ class HotPath:
             sc = P["scal"].cpu().numpy()
             return dict(y=P["y"].cpu().numpy(), dx=P["dx"].cpu().numpy(), r=P["r"].cpu().numpy(), ssqrNew=float(sc[0]),
                         ssqrdx=float(sc[1]), alpha=float(sc[2]), normr=float(sc[3]))
+
+    def pcg(self, rv: np.ndarray, rb: np.ndarray | None = None, y0: float = 1.0, cgpars: dict | None = None):
+        """The search direction of wrapPcg.m:43-130 on the device: the direct step, then loopPcg refinement while
+        |r|_inf >= y0 * cgpars["restol"].  Valid after blkchol (and deninfac with dense columns) for LP, Lorentz and PSD
+        cones; the scaling is the one set_scaling uploaded last (with d.auxdet, d.auxtr when there are Lorentz cones).
+        rv: N = K.l + sum(K.q) + sum(K.s.^2) in x-space, rb: m or None; cgpars: any of restol, stagtol, maxiter, refine,
+        qprec (defaults: checkpars.m).  Returns dict(y, dx, r, k, stop, trials, normr) as host arrays / numbers.
+        Raises SB200Error while the library stream is being captured: the loop reads its status back on the host."""
+        t = self.torch
+        L = lib()
+        N = self.lpN + self.nq + self.qdim + self.lenud
+        cg = dict(CgPars.DEFAULTS, **(cgpars or {}))
+        pars = CgPars(cg["restol"], cg["stagtol"], int(cg["maxiter"]), int(cg["refine"]), int(cg["qprec"]))
+        P = getattr(self, "_pcgf", None)
+        st = _PcgStatus()
+        with t.cuda.stream(self.stream()):
+            if t.cuda.is_current_stream_capturing():
+                # nothing may be enqueued into the capture: let the entry refuse before any upload
+                cones = _PcgCones(self.nq, self.qdim, None, None, None, None, None, None, self.nden, None, None, 0)
+                check(L.sb200_wrappcg_full_dev(self.ada, self.psd, self.chol, self.dpr1, C.byref(cones), C.byref(pars),
+                                               *([None] * 8), C.c_double(y0), None, None, None, C.byref(st), None), "wrappcg_full")
+            rv = np.ascontiguousarray(np.asarray(rv, dtype=np.float64).ravel())
+            assert rv.size == N, (rv.size, N)
+            if P is None:
+                f64 = dict(dtype=t.float64, device=self.dev)
+                nw = int(L.sb200_wrappcg_full_work(I64(N), I64(self.m), I64(self.nq), I64(self.qdim)))
+                P = self._pcgf = dict(work=t.zeros(nw, **f64), y=t.zeros(self.m, **f64), dx=t.zeros(N, **f64),
+                                      r=t.zeros(self.m, **f64), rv=t.zeros(N, **f64), rb=t.zeros(self.m, **f64))
+            P["rv"].copy_(t.from_numpy(rv))
+            if rb is not None:
+                P["rb"].copy_(t.from_numpy(np.ascontiguousarray(np.asarray(rb, dtype=np.float64).ravel())))
+            nq = self.nq
+            cones = _PcgCones(nq, self.qdim, _p(self.qbs) if nq else None, _p(self.d_det), _p(self.d_q1), _p(self.d_q2),
+                              _p(self.d_auxdet), _p(self.d_auxtr), self.nden, _p(self.den_idx) if self.nden else None,
+                              _p(self.Ad) if self.nden else None, 0)
+            check(L.sb200_wrappcg_full_dev(self.ada, self.psd, self.chol, self.dpr1, C.byref(cones), C.byref(pars), _p(self.d_l),
+                                           _p(self.d_u), _p(self.d_perm) if self.has_perm else None, _p(self.Lrect),
+                                           _p(self.dvec_den if self.nden else self.dvec), _p(self.flag), _p(P["rv"]),
+                                           _p(P["rb"]) if rb is not None else None, C.c_double(y0), _p(P["y"]), _p(P["dx"]),
+                                           _p(P["r"]), C.byref(st), _p(P["work"])), "wrappcg_full")
+            self.sync()
+            return dict(y=P["y"].cpu().numpy(), dx=P["dx"].cpu().numpy(), r=P["r"].cpu().numpy(), k=int(st.k), stop=int(st.stop),
+                        trials=int(st.trials), normr=float(st.normr))
 
     def profile(self, nsolve=4, npsdscale=12, sharded=False, reps=3):
         """Per-kernel device time of one iteration, averaged over `reps`: {kernel name: (launches, ms)}.  An event is
